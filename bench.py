@@ -10,6 +10,7 @@ them under `configs`, each with its own roofline entry.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload nested|flat|blob|mixed] [--items M]
   python bench.py --impl reference ...      (the CPU path: oracle port on all host cores, same items)
+  python bench.py ... --dump-outputs DIR    (a seeded sample of what the last timed step returned, as .npy files)
 
 Under torchrun (N > 1) every rank owns one GPU and its own shard of the batch (items shard by
 index, no collective on the data path); rank 0 prints one JSON line.
@@ -257,6 +258,10 @@ def run_reference(args, rank, world):
         t_sum += t
         last = (req, rep)
     req, rep = last
+    if args.dump_outputs:
+        sides = {} if req is None else {"request": (req[1], req[2], req[0].__getitem__)}
+        sides["reply"] = (rep[1], rep[2], rep[0].__getitem__)
+        dump_outputs(args.dump_outputs, sides)
     J_in = int(len(wl.req_json)) if wl.req_json is not None else 0
     W_out = int(req[1][n]) if req is not None else 0
     value = n * args.steps / t_sum
@@ -272,6 +277,32 @@ def run_reference(args, rank, world):
         "wall_s": time.perf_counter() - t0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_SEED = 0xD0B5
+DUMP_ITEMS = 4096
+DUMP_BYTES = 7 << 20  # output bytes per direction: two directions of float32 bytes stay under 64 MB
+
+
+def dump_outputs(directory, sides):
+    """--dump-outputs: for each direction {name: (output offsets[n + 1], status[n], gather)}, the items of a fixed seeded
+    permutation of the batch (at most DUMP_ITEMS, while their output bytes fit DUMP_BYTES), written as
+    <name>_items (index in the batch), <name>_status, <name>_lengths and <name>_bytes (their outputs, concatenated).
+    gather(idx) returns the output bytes at the byte positions idx.  Two builds fed the same arguments dump the same
+    items unless their output lengths differ."""
+    os.makedirs(directory, exist_ok=True)
+    for name, (out_off, status, gather) in sides.items():
+        off = np.asarray(out_off).astype(np.int64)
+        lens = np.diff(off)
+        order = np.random.default_rng(DUMP_SEED).permutation(len(lens))[:DUMP_ITEMS]
+        items = np.sort(order[np.cumsum(lens[order]) <= DUMP_BYTES])
+        ln = lens[items]
+        idx = np.repeat(off[items] - np.cumsum(ln) + ln, ln) + np.arange(int(ln.sum()), dtype=np.int64)
+        data = np.asarray(gather(idx), np.uint8)
+        arrays = {"items": items.astype(np.float64), "status": np.asarray(status)[items].astype(np.float32),
+                  "lengths": ln.astype(np.float64), "bytes": data.astype(np.float32)}
+        for k, a in arrays.items():
+            np.save(os.path.join(directory, "%s_%s.npy" % (name, k)), a)
 
 
 def digest(*arrays):
@@ -353,6 +384,17 @@ class Resident:
         e1.record(self.stream)
         barrier()
         return e0.elapsed_time(e1)
+
+    def outputs(self):
+        """what the last step returned, per direction, in the form dump_outputs takes"""
+        torch, dev = self.torch, self.dev
+
+        def side(out, off, st):
+            return (off.cpu().numpy(), st.cpu().numpy(), lambda idx: out[torch.from_numpy(idx).to(dev)].cpu().numpy())
+
+        sides = {"request": side(self.d_req_out, self.d_req_out_off, self.d_req_st)} if self.have_req else {}
+        sides["reply"] = side(self.d_rep_out, self.d_rep_out_off, self.d_rep_st)
+        return sides
 
     def kernel_table(self):
         """per-kernel device time: the same kernels, same inputs, serialized on one stream so that each launch has the
@@ -476,7 +518,11 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the whole-batch comparison with the CPU oracle")
     ap.add_argument("--e2e-serial", action="store_true", help="end-to-end: request call, then reply call (default: both in flight)")
     ap.add_argument("--one-stream", action="store_true", help="serialize request and reply side on one stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of what the last step "
+                                                          "returned to DIR/<name>.npy (float32 / float64, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.items == 0:
         args.items = DEFAULT_ITEMS[args.workload]
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -533,6 +579,8 @@ def main():
     ms = R.timed(args.steps, barrier, args.one_stream)
     clocks = sampler.stop()
     launches = eng.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, R.outputs())
     ms_max = max_ranks(ms)
     value = world * n * args.steps / (ms_max / 1000.0)
     kern = R.kernel_table()

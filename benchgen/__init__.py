@@ -25,7 +25,8 @@ def build(force=False):
 def _load():
     global _lib
     if _lib is None:
-        build()
+        if not os.path.exists(LIB):  # build() keeps it current; loading never writes into a built tree
+            build()
         L = C.CDLL(LIB)
         vp = C.c_void_p
         L.ggr_gen_flat.argtypes = [C.c_uint64, C.c_int64, vp, C.c_uint64, vp, vp, C.c_uint64, vp]
